@@ -8,7 +8,7 @@ eval-mode BatchNorm, forward only, on a batch of synthetic dental-arch clouds of
     FPS 24000->1024  ->  ball query (r=0.1, K=32)  ->  fused gather+MLP(9->32->32->64)+max.
 metric = sampled points per second = clouds * 1024 / time, whole job (all ranks).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--clouds B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--clouds B] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 * ``value``: the PUBLIC module call ``sa(xyz, feats)`` with inputs resident in HBM, CUDA-event timed, max over ranks.
@@ -26,6 +26,10 @@ metric = sampled points per second = clouds * 1024 / time, whole job (all ranks)
 * ``cpu_baseline`` / ``--impl reference``: the oracle's port of the reference's CPU-capable formulation of the same
   path (FPS loop + query_ball_point + grouped MLP, one cloud per host thread), bounded sample.
 Inputs are larger than L2 (B*24000*6*4 bytes = 682 MB at the default B = 1184); no explicit flush.
+* ``--dump-outputs DIR``: after the timed steps, rank 0 writes what the last timed ``sa(xyz, feats)`` returned, for the same
+  seeded sample of at most ``DUMP_CLOUDS`` clouds every run, as float32 ``DIR/new_xyz.npy`` (n, 3, 1024) and
+  ``DIR/new_points.npy`` (n, 64, 1024), with the cloud indices in ``DIR/cloud_index.npy`` (float64): so that two builds can be
+  compared output for output.  The inputs depend only on the arguments.
 """
 from __future__ import annotations
 
@@ -51,6 +55,7 @@ UNIT = "sampled points/s"
 WORKLOAD = "pointnet++ SA1 forward: FPS 24000->1024, ball query r=0.1 K=32, group-MLP 9->[32,32,64], eval BN"
 MLP_FLOP_PER_CLOUD = 2.0 * NPOINT * NSAMPLE * (9 * 32 + 32 * 32 + 32 * 64)      # SURVEY.md 8d: 0.220 GFLOP
 B200_FP32_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12                                  # CUDA-core FMA peak at max clock
+DUMP_CLOUDS = 128                     # 128 * (3 + 64) * 1024 * 4 bytes = 35 MB of dumped outputs at most
 
 
 def host_cores() -> int:
@@ -251,6 +256,17 @@ def time_cpu(layers, sample_clouds: int, steps: int, warmup: int):
     return sample_clouds * NPOINT / dt, dt, cores
 
 
+def dump_outputs(out_dir: str, new_xyz: torch.Tensor, new_points: torch.Tensor) -> None:
+    """A fixed, seeded sample of the clouds of one step's outputs, as float32 .npy files (see the module docstring)."""
+    B = new_xyz.shape[0]
+    pick = np.sort(np.random.default_rng(0).choice(B, size=min(B, DUMP_CLOUDS), replace=False))
+    index = torch.from_numpy(pick).to(new_xyz.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "new_xyz.npy"), new_xyz.index_select(0, index).float().cpu().numpy())
+    np.save(os.path.join(out_dir, "new_points.npy"), new_points.index_select(0, index).float().cpu().numpy())
+    np.save(os.path.join(out_dir, "cloud_index.npy"), pick.astype(np.float64))
+
+
 def elementwise_rel(a: torch.Tensor, b: torch.Tensor, floor: float = 0.05) -> float:
     a, b = a.double(), b.double()
     return float(((a - b).abs() / b.abs().clamp(min=floor * float(b.abs().max()) + 1e-300)).max())
@@ -276,7 +292,11 @@ def main():
     ap.add_argument("--fps-mode", type=int, default=0, help="0 auto; 100*G+CS resident shape, -2 bucket, -(10+W) bucket with W warps per cloud (experiments)")
     ap.add_argument("--ball-path", type=int, default=0, help="0 auto, 4 index-order tile scan, 8 uniform grid (experiments)")
     ap.add_argument("--sa-engine", type=int, default=0, help="0 auto, 1 fp32 CUDA cores, 2 tcgen05 (experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's outputs to DIR as .npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     from toothgroupnetwork_b200 import sharding
@@ -372,10 +392,13 @@ def main():
         with ClockSampler(local) as clk:
             t_start.record()
             for s in range(args.steps):
-                sa(xyz, feats)
+                last = sa(xyz, feats)
             t_end.record()
             torch.cuda.synchronize()
         launches = L.launch_count() - launches0
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, *last)
+        del last
         sharding.barrier()
         # stage breakdown: the same kernels with events between the stages (not part of `value`)
         stage_events = [[ev() for _ in range(4)] for _ in range(min(args.steps, 5))]

@@ -7,7 +7,8 @@ verbatim for sm_100a into oracle/_ref/libpointops_ref.so by ``make -C oracle ref
 Inputs are regenerated from seeds by the tests (toothgroupnetwork_b200.clouds), only the reference
 outputs are stored.  These fixtures pin the CPU oracle (tests/test_oracle_golden.py) against the
 real kernels: FPS indices + final running minima, kNN indices + squared distances (bitwise), the
-gather-family forwards (bitwise).
+gather-family forwards (bitwise).  The large kNN and gather outputs are stored as digests with a sample
+(oracle/golden.pack).
 """
 import os
 import sys
@@ -17,7 +18,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
-from oracle import ref_cuda  # noqa: E402
+from oracle import golden, ref_cuda  # noqa: E402
 from toothgroupnetwork_b200 import clouds  # noqa: E402
 
 FPS_CASES = {
@@ -75,7 +76,7 @@ def main(out_dir):
                                     torch.tensor(noffs, dtype=torch.int32).cuda())
         fix[f"{name}_idx"] = idx.cpu().numpy()
         fix[f"{name}_d2"] = d2.cpu().numpy()
-    np.savez_compressed(os.path.join(out_dir, "ref_cuda_knn.npz"), **fix)
+    np.savez_compressed(os.path.join(out_dir, "ref_cuda_knn.npz"), **{e: v for k, a in fix.items() for e, v in golden.pack(k, a).items()})
 
     # gather family forwards on seeded random tensors
     g = torch.Generator().manual_seed(0)
@@ -94,7 +95,7 @@ def main(out_dir):
         "subtraction": ref_cuda.subtraction_forward(inp.cuda(), in2.cuda(), idxn.cuda()).cpu().numpy(),
         "aggregation": ref_cuda.aggregation_forward(inp.cuda(), pos.cuda(), wgt.cuda(), idxn.cuda()).cpu().numpy(),
     }
-    np.savez_compressed(os.path.join(out_dir, "ref_cuda_gather.npz"), **fix)
+    np.savez_compressed(os.path.join(out_dir, "ref_cuda_gather.npz"), **{e: v for k, a in fix.items() for e, v in golden.pack(k, a).items()})
     for f in sorted(os.listdir(out_dir)):
         print(f, os.path.getsize(os.path.join(out_dir, f)))
 

@@ -77,5 +77,10 @@ def test_dbscan_class_refuses_what_it_does_not_implement():
         clustering.DBSCAN(eps=0.1, min_samples=3, metric="manhattan")
     with pytest.raises(clustering.L.TgnError):
         clustering.DBSCAN(eps=0.1, min_samples=3).fit(np.zeros((4, 2), np.float32))
+    pts = np.zeros((4, 3), np.float32)
+    if torch.cuda.is_available():                                    # the same call on a GPU runs there
+        from sklearn.cluster import DBSCAN
+        assert np.array_equal(clustering.DBSCAN(eps=0.1, min_samples=3).fit(pts).labels_, DBSCAN(eps=0.1, min_samples=3).fit(pts).labels_)
+        return
     with pytest.raises(clustering.L.TgnError):                        # no CPU path: the product fails loudly without a GPU
-        clustering.DBSCAN(eps=0.1, min_samples=3).fit(np.zeros((4, 3), np.float32))
+        clustering.DBSCAN(eps=0.1, min_samples=3).fit(pts)

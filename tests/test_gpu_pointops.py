@@ -1,18 +1,34 @@
 """GPU parity of the pointops side (FPS, kNN, gather family) -- bit-exact for indices and
 forward values -- against (a) the CPU oracle and (b) the reference's own kernels compiled
-verbatim (oracle/_ref), on seeded inputs."""
+verbatim (oracle/_ref), on seeded inputs.  The reference kernels' outputs are stored in tests/golden/ref_live_pointops.npz
+(oracle/golden.py: recorded by a run with TGN_GOLDEN_RECORD set where oracle/_ref is built)."""
 import ctypes
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import oracle, ref_cuda
+from oracle import golden, oracle, ref_cuda
 from toothgroupnetwork_b200 import _lib as L
 from toothgroupnetwork_b200 import clouds, pointops, pointops_cuda
 
 pytestmark = pytest.mark.gpu
-needs_ref = pytest.mark.skipif(not ref_cuda.available(), reason="oracle/_ref not built")
+G = golden.Golden("ref_live_pointops")
+
+
+def assert_exact(key, got, compute):
+    assert G.exact(key, got, compute), f"{key}: {G.mismatch(key, got)}"
+
+
+def reference(call):
+    """the reference kernel's outputs, computed once and only when they are recorded: reference(call)(i) -> output i"""
+    out = []
+
+    def get(i):
+        if not out:
+            out.extend(call())
+        return out[i]
+    return get
 
 
 def dev(a, dtype=None):
@@ -69,20 +85,19 @@ def test_fps_matches_oracle(name, build, ms, mode):
     assert np.array_equal(got.cpu().numpy(), want)
 
 
-@needs_ref
 @pytest.mark.parametrize("name,build,ms", FPS_CASES, ids=[c[0] for c in FPS_CASES])
 def test_fps_matches_reference_kernel(name, build, ms):
     cl = build()
     xyz, offset, new_offset = _pack(cl, ms)
     n_max = max(c.shape[0] for c in cl)
     x, o, no = xyz.cuda(), i32(offset), i32(new_offset)
-    ref_idx, ref_tmp = ref_cuda.furthestsampling(x, o, no, n_max, int(new_offset[-1]))
+    ref = reference(lambda: ref_cuda.furthestsampling(x, o, no, n_max, int(new_offset[-1])))
     got = pointops.furthestsampling(x, o, no)
-    assert torch.equal(got, ref_idx)
+    assert_exact(f"fps_{name}_idx", got, lambda: ref(0))
     # the oracle reproduces the reference kernel too (idx AND the final running minima, bitwise)
     o_idx, o_tmp = oracle.furthestsampling(xyz.numpy(), offset, new_offset, return_tmp=True)
-    assert np.array_equal(o_idx, ref_idx.cpu().numpy())
-    assert np.array_equal(o_tmp.view(np.uint32), ref_tmp.cpu().numpy().view(np.uint32))
+    assert_exact(f"fps_{name}_idx", o_idx, lambda: ref(0))
+    assert_exact(f"fps_{name}_tmp", o_tmp, lambda: ref(1))
 
 
 def test_fps_drop_in_launcher_and_tmp_writeback():
@@ -157,17 +172,17 @@ def test_knn_matches_oracle(name, build, m, off, noff, k):
     assert np.array_equal(dist.cpu().numpy().view(np.uint32), w_dist.view(np.uint32))
 
 
-@needs_ref
 @pytest.mark.parametrize("name,build,m,off,noff,k", KNN_CASES, ids=[c[0] for c in KNN_CASES])
 def test_knn_matches_reference_kernel(name, build, m, off, noff, k):
     xyz, new_xyz, off, noff = _knn_inputs(build, m, off, noff)
     x, q, o, no = xyz.cuda(), new_xyz.cuda(), i32(off), i32(noff)
-    r_idx, r_d2 = ref_cuda.knnquery(k, x, q, o, no)
+    ref = reference(lambda: ref_cuda.knnquery(k, x, q, o, no))
     idx, d2 = pointops.knn_packed(k, x, q, o, no)
-    assert torch.equal(d2.view(torch.int32), r_d2.view(torch.int32))
-    assert torch.equal(idx, r_idx)
+    assert_exact(f"knn_{name}_d2", d2, lambda: ref(1))              # float32, bit for bit
+    assert_exact(f"knn_{name}_idx", idx, lambda: ref(0))
     w_idx, _, w_d2 = oracle.knnquery(k, xyz.numpy(), new_xyz.numpy(), off, noff)
-    assert np.array_equal(w_idx, r_idx.cpu().numpy()) and np.array_equal(w_d2.view(np.uint32), r_d2.cpu().numpy().view(np.uint32))
+    assert_exact(f"knn_{name}_idx", w_idx, lambda: ref(0))
+    assert_exact(f"knn_{name}_d2", w_d2, lambda: ref(1))
 
 
 GRID_CASES = [
@@ -191,7 +206,7 @@ GRID_CASES = [
 @pytest.mark.parametrize("name,build,off,qbuild,noff,k", GRID_CASES, ids=[c[0] for c in GRID_CASES])
 def test_knn_grid_equals_bruteforce_kernel_and_reference(name, build, off, qbuild, noff, k):
     """The uniform-grid search (csrc/knn_grid.cu) against the brute-force warp kernel (csrc/knn.cu), bit for bit --
-    indices including the reference's tie order -- and against the verbatim reference kernel when it is present."""
+    indices including the reference's tie order -- and against the verbatim reference kernel."""
     xyz = build().contiguous()
     q = xyz if qbuild is None else qbuild(xyz).contiguous()
     o, no = i32(np.asarray(off, np.int32)), i32(np.asarray(off if noff is None else noff, np.int32))
@@ -215,9 +230,9 @@ def test_knn_grid_equals_bruteforce_kernel_and_reference(name, build, off, qbuil
     assert L.launch_count() - launches == 1
     kk = min(k, k2)
     assert torch.equal(h_idx[:, :kk], b_idx[:, :kk]) or name.startswith(("duplicated", "all_points"))
-    if ref_cuda.available():
-        r_idx, r_d2 = ref_cuda.knnquery(k, x, qq, o, no)
-        assert torch.equal(g_d2.view(torch.int32), r_d2.view(torch.int32)) and torch.equal(g_idx, r_idx)
+    ref = reference(lambda: ref_cuda.knnquery(k, x, qq, o, no))
+    assert_exact(f"knn_grid_{name}_d2", g_d2, lambda: ref(1))
+    assert_exact(f"knn_grid_{name}_idx", g_idx, lambda: ref(0))
     x.add_(0.0)                                                   # in-place write bumps the version: caches must miss
     launches = L.launch_count()
     pointops.knn_packed(k, x, qq if qbuild is not None else x, o, no)
@@ -251,8 +266,7 @@ def test_grouping_forward_backward(c):
     out.backward(go.cuda())
     want = oracle.grouping_backward(go.numpy(), idx.numpy(), n)
     np.testing.assert_allclose(x.grad.cpu().numpy(), want, rtol=1e-5, atol=1e-5)
-    if ref_cuda.available():
-        assert torch.equal(out.detach(), ref_cuda.grouping_forward(inp.cuda(), idx.cuda()))
+    assert_exact(f"grouping_{c}", out, lambda: ref_cuda.grouping_forward(inp.cuda(), idx.cuda()))
 
 
 def test_interpolation_kernels():
@@ -267,8 +281,7 @@ def test_interpolation_kernels():
     gi = torch.zeros(m, c, device="cuda")
     pointops_cuda.interpolation_backward_cuda(n, c, k, go.cuda(), idx.cuda(), w.cuda(), gi)
     np.testing.assert_allclose(gi.cpu().numpy(), oracle.interpolation_backward(go.numpy(), idx.numpy(), w.numpy(), m), rtol=1e-4, atol=1e-5)
-    if ref_cuda.available():
-        assert torch.equal(out, ref_cuda.interpolation_forward(inp.cuda(), idx.cuda(), w.cuda()))
+    assert_exact("interpolation", out, lambda: ref_cuda.interpolation_forward(inp.cuda(), idx.cuda(), w.cuda()))
 
 
 @pytest.mark.parametrize("c", [32, 6])
@@ -284,8 +297,7 @@ def test_subtraction(c):
     g1, g2 = oracle.subtraction_backward(idx.numpy(), go.numpy())
     np.testing.assert_allclose(x1.grad.cpu().numpy(), g1, rtol=1e-4, atol=1e-5)
     np.testing.assert_allclose(x2.grad.cpu().numpy(), g2, rtol=1e-4, atol=1e-5)
-    if ref_cuda.available():
-        assert torch.equal(out.detach(), ref_cuda.subtraction_forward(a.cuda(), b.cuda(), idx.cuda()))
+    assert_exact(f"subtraction_{c}", out, lambda: ref_cuda.subtraction_forward(a.cuda(), b.cuda(), idx.cuda()))
 
 
 def test_aggregation():
@@ -302,8 +314,7 @@ def test_aggregation():
     np.testing.assert_allclose(ti.grad.cpu().numpy(), gi, rtol=1e-4, atol=1e-4)
     np.testing.assert_allclose(tp.grad.cpu().numpy(), gp, rtol=1e-5, atol=1e-6)
     np.testing.assert_allclose(tw.grad.cpu().numpy(), gw, rtol=1e-4, atol=1e-4)
-    if ref_cuda.available():
-        assert torch.equal(out.detach(), ref_cuda.aggregation_forward(inp.cuda(), pos.cuda(), w.cuda(), idx.cuda()))
+    assert_exact("aggregation", out, lambda: ref_cuda.aggregation_forward(inp.cuda(), pos.cuda(), w.cuda(), idx.cuda()))
 
 
 def test_queryandgroup_and_interpolation_composites():

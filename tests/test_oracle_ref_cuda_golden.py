@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import oracle
+from oracle import golden, oracle
 
 _spec = importlib.util.spec_from_file_location("make_ref_cuda_golden",
                                                os.path.join(os.path.dirname(__file__), "golden", "make_ref_cuda_golden.py"))
@@ -34,7 +34,7 @@ def test_fps_oracle_equals_reference_kernel(golden_dir, name):
 
 @pytest.mark.parametrize("name", sorted(gen.KNN_CASES))
 def test_knn_oracle_equals_reference_kernel(golden_dir, name):
-    fix = _load(golden_dir, "ref_cuda_knn.npz")
+    fix = golden.Golden("ref_cuda_knn", record=False)
     kind, n, seed, offs, qcounts, k = gen.KNN_CASES[name]
     xyz = gen.make_cloud(kind, n, seed)
     if qcounts is None:
@@ -44,12 +44,12 @@ def test_knn_oracle_equals_reference_kernel(golden_dir, name):
         q = torch.cat([xyz[s:s + c] for s, c in zip(starts, qcounts)], 0)
         noffs = list(np.cumsum(qcounts))
     idx, _, d2 = oracle.knnquery(k, xyz.numpy(), q.numpy(), np.asarray(offs, np.int32), np.asarray(noffs, np.int32))
-    assert np.array_equal(d2.view(np.uint32), fix[f"{name}_d2"].view(np.uint32))
-    assert np.array_equal(idx, fix[f"{name}_idx"])
+    assert fix.exact(f"{name}_d2", d2, None), fix.mismatch(f"{name}_d2", d2)          # float32, bit for bit
+    assert fix.exact(f"{name}_idx", idx, None), fix.mismatch(f"{name}_idx", idx)
 
 
 def test_gather_family_oracle_equals_reference_kernels(golden_dir):
-    fix = _load(golden_dir, "ref_cuda_gather.npz")
+    fix = golden.Golden("ref_cuda_gather", record=False)
     g = torch.Generator().manual_seed(0)
     n, m, k, c, w_c = 1500, 400, 16, 32, 4
     inp = torch.randn(n, c, generator=g)
@@ -60,8 +60,8 @@ def test_gather_family_oracle_equals_reference_kernels(golden_dir):
     idxn = torch.randint(0, n, (n, k), generator=g, dtype=torch.int32)
     pos = torch.randn(n, k, c, generator=g)
     wgt = torch.randn(n, k, w_c, generator=g)
-    eq = lambda a, b: np.array_equal(np.asarray(a).view(np.uint32), np.asarray(b).view(np.uint32))
-    assert eq(oracle.grouping_forward(inp.numpy(), idx.numpy()), fix["grouping"])
-    assert eq(oracle.interpolation_forward(inp.numpy(), idx3.numpy(), w3.numpy()), fix["interpolation"])
-    assert eq(oracle.subtraction_forward(inp.numpy(), in2.numpy(), idxn.numpy()), fix["subtraction"])
-    assert eq(oracle.aggregation_forward(inp.numpy(), pos.numpy(), wgt.numpy(), idxn.numpy()), fix["aggregation"])
+    for key, got in (("grouping", oracle.grouping_forward(inp.numpy(), idx.numpy())),
+                     ("interpolation", oracle.interpolation_forward(inp.numpy(), idx3.numpy(), w3.numpy())),
+                     ("subtraction", oracle.subtraction_forward(inp.numpy(), in2.numpy(), idxn.numpy())),
+                     ("aggregation", oracle.aggregation_forward(inp.numpy(), pos.numpy(), wgt.numpy(), idxn.numpy()))):
+        assert fix.exact(key, got, None), (key, fix.mismatch(key, got))                   # float32, bit for bit
