@@ -114,6 +114,21 @@ int tgn_knn_grid_build(int b, int n_total, const float *xyz, const int *offset, 
 int tgn_knn_grid_query(int b, int n_total, int m, int nsample, const float *xyz, const float *new_xyz, const int *offset,
                        const int *new_offset, const void *workspace, int *idx, float *dist2, void *stream);
 
+/* Exact float64 kNN with scikit-learn KDTree semantics: replaces the host KDTree searches of the tgnet boundary stage
+ * (inference_pipeline_tgn.py:289-330, :107-140).  points (n,3) and queries (m,3) float64 DEVICE; for every query the k <= 64
+ * (and k <= n) nearest points in ascending (rdist, index) order, rdist = (dx*dx + dy*dy) + dz*dz in float64 without FMA
+ * contraction; exact ties come out lower index first.  Build once per point set into a caller-owned DEVICE workspace of
+ * tgn_knn_f64_bytes(n) bytes (it holds the grid of tgn_knn_grid_build plus a float64 copy of the points in cell order) and
+ * reuse it for every query set and k.  Outputs, each optional (NULL = not written): idx (m,k) int64, dist (m,k) float64 =
+ * sqrt(rdist) correctly rounded.  With labels (n) float64 the query also writes nearest_label (m) = labels[idx[:,0]],
+ * is_boundary (m) bytes = (count / k < ratio) with count the neighbours whose label equals nearest_label, and the number
+ * of boundary queries to the DEVICE int n_boundary (zeroed by the call); no (m,k) matrix is needed for that. */
+size_t tgn_knn_f64_bytes(int n);
+int tgn_knn_f64_build(int n, const double *points, void *workspace, void *stream);
+int tgn_knn_f64_query(int n, int m, int k, const double *queries, const void *workspace, int64_t *idx, double *dist,
+                      const double *labels, double ratio, double *nearest_label, unsigned char *is_boundary, int *n_boundary,
+                      void *stream);
+
 int tgn_grouping_forward(int m, int nsample, int c, const float *input, const int *idx, float *output, void *stream);
 int tgn_grouping_backward(int m, int nsample, int c, const float *grad_output, const int *idx, float *grad_input, void *stream);
 int tgn_interpolation_forward(int n, int c, int k, const float *input, const int *idx, const float *weight, float *output, void *stream);

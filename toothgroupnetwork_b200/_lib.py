@@ -29,6 +29,8 @@ _SIGS = {
     "tgn_weighted_gather_backward_det": [ctypes.c_longlong, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp],
     "tgn_knn_grid_build": [_i, _i, _vp, _vp, _vp, _vp],
     "tgn_knn_grid_query": [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tgn_knn_f64_build": [_i, _vp, _vp, _vp],
+    "tgn_knn_f64_query": [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, ctypes.c_double, _vp, _vp, _vp, _vp],
     "tgn_grouping_forward": [_i, _i, _i, _vp, _vp, _vp, _vp],
     "tgn_grouping_backward": [_i, _i, _i, _vp, _vp, _vp, _vp],
     "tgn_interpolation_forward": [_i, _i, _i, _vp, _vp, _vp, _vp, _vp],
@@ -108,7 +110,8 @@ REFERENCE_LAUNCHERS = [
     "subtraction_forward_cuda_launcher", "subtraction_backward_cuda_launcher",
     "aggregation_forward_cuda_launcher", "aggregation_backward_cuda_launcher",
 ]
-EXPORTS = list(_SIGS) + REFERENCE_LAUNCHERS + ["tgn_version", "tgn_last_error", "tgn_launch_count", "tgn_pw_packed_bytes", "tgn_pw_struct_size", "tgn_knn_grid_bytes", "tgn_csr_bytes", "tgn_pt_layer_struct_size", "tgn_dbscan_bytes"]
+EXPORTS = list(_SIGS) + REFERENCE_LAUNCHERS + ["tgn_version", "tgn_last_error", "tgn_launch_count", "tgn_pw_packed_bytes", "tgn_pw_struct_size", "tgn_knn_grid_bytes", "tgn_csr_bytes", "tgn_pt_layer_struct_size", "tgn_dbscan_bytes",
+                                                  "tgn_knn_f64_bytes"]
 
 
 class TgnError(RuntimeError):
@@ -139,6 +142,8 @@ def load() -> ctypes.CDLL:
     lib.tgn_knn_grid_bytes.argtypes = [_i, _i]
     lib.tgn_knn_grid_bytes.restype = ctypes.c_size_t
     lib.tgn_dbscan_bytes.argtypes = [_i]
+    lib.tgn_knn_f64_bytes.argtypes = [_i]
+    lib.tgn_knn_f64_bytes.restype = ctypes.c_size_t
     lib.tgn_dbscan_bytes.restype = ctypes.c_size_t
     lib.tgn_pw_struct_size.argtypes = [_i]
     lib.tgn_pw_struct_size.restype = _i

@@ -19,7 +19,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_lib")
 LIB = os.path.join(OUT_DIR, "libtgn_b200.so")
-SOURCES = ["lib.cu", "fps.cu", "fps_bucket.cu", "knn.cu", "knn_grid.cu", "crop_knn.cu", "gather.cu", "csr.cu", "ballquery.cu", "ballquery_grid.cu", "sa_mlp.cu", "sa_mlp_tc.cu", "sa_mlp_tc8.cu", "sa_mlp_tcw.cu", "pw_mlp.cu", "pt_layer.cu", "dbscan.cu"]
+SOURCES = ["lib.cu", "fps.cu", "fps_bucket.cu", "knn.cu", "knn_grid.cu", "crop_knn.cu", "gather.cu", "csr.cu", "ballquery.cu", "ballquery_grid.cu", "sa_mlp.cu", "sa_mlp_tc.cu", "sa_mlp_tc8.cu", "sa_mlp_tcw.cu", "pw_mlp.cu", "pt_layer.cu", "dbscan.cu", "knn_f64.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC",

@@ -77,6 +77,18 @@ def accelerate_blocks(blocks_module=None) -> None:
     blocks_fused.accelerate(blocks_module)
 
 
+def accelerate_inference_tgn(module=None) -> None:
+    """Optional: run the boundary stage of the reference's tgnet inference pipeline on the GPU -- its
+    ``InferencePipeLine.get_boundary_sampled_feats`` (inference_pipeline_tgn.py:289-330: KDTree k = 40 label vote,
+    uniform + FPS resampling) and the module's other ``KDTree`` searches (:107-140), see
+    ``toothgroupnetwork_b200.boundary``.  Imports ``inference_pipelines.inference_pipeline_tgn`` from ``sys.path`` when
+    no module is passed."""
+    from . import boundary
+    if module is None:
+        module = importlib.import_module("inference_pipelines.inference_pipeline_tgn")
+    boundary.accelerate_inference_pipeline(module)
+
+
 def uninstall() -> None:
     for alias in _TARGETS:
         sys.modules.pop(alias, None)
